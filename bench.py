@@ -1,6 +1,7 @@
 """bench.py -- SpKBGAT fwd+bwd edges/sec on synthetic power-law KGs (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c4|c5] [--impl reference]
+                  [--dump-outputs DIR]
 
 A step = SpKBGATModified forward (2 attention layers) + loss.backward() over the whole graph, loss =
 <out_entity, G_e> + <out_relation, G_r> (SURVEY.md 8d), batch_entities = arange(N) (dense mask).
@@ -11,6 +12,9 @@ A step = SpKBGATModified forward (2 attention layers) + loss.backward() over the
 `roofline`: the dominant kernel's algorithmic bytes / its CUDA-event time, against MEASURED_PEAKS.json.
 `cpu_baseline`: the CPU port of the reference path (oracle/ref_torch.py, COO sparse.sum like the reference)
             on a bounded sample, host cores of this box.
+--dump-outputs DIR writes what the last timed step handed to its caller (outputs, loss, parameter gradients) as
+            DIR/<name>.npy; inputs are seeded, so two builds run with the same arguments can be compared array by array.
+The benchmark writes nothing into the source tree (it may be read-only).
 """
 import argparse
 import json
@@ -20,6 +24,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True        # no __pycache__ in the source tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -174,9 +179,10 @@ def describe(workload):
             f"heads=[{HEADS},{HEADS}] rows: {int(100 * h_)}% Pareto(alpha={a_}) hubs + uniform")
 
 
-def run_config(workload, world, rank, dev, steps, warmup, want_prof=False, want_e2e=False, clocks=False):
+def run_config(workload, world, rank, dev, steps, warmup, want_prof=False, want_e2e=False, clocks=False, dump_dir=None):
     """Builds the runner for `workload`, runs `warmup` untimed + `steps` timed steps (CUDA events, barrier + synchronize on
-    both sides, max over ranks). Returns a dict; the runner is released before returning."""
+    both sides, max over ranks). With `dump_dir`, what the last timed step computed is written there (dump_outputs) before
+    anything else runs. Returns a dict; the runner is released before returning."""
     import torch.distributed as dist
     from recon_b200 import _lib, profiler
     add_workload(workload)
@@ -205,12 +211,15 @@ def run_config(workload, world, rank, dev, steps, warmup, want_prof=False, want_
     l0 = _lib.launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
-    for _ in range(steps):
+    for i in range(steps):
+        runner.keep_outputs = dump_dir is not None and i == steps - 1
         runner.step()
     ev1.record()
     barrier()
     res = {"workload": workload, "e_total": e_total, "launches": _lib.launch_count() - l0,
            "peak_mem_gb": round(torch.cuda.max_memory_allocated() / 2 ** 30, 1)}
+    if dump_dir is not None:
+        res["dump"] = dump_outputs(runner, dump_dir)
     ms = ev0.elapsed_time(ev1) / steps
     res["clocks"] = sampler.stop() if sampler else None
     if world > 1:
@@ -260,6 +269,37 @@ def run_config(workload, world, rank, dev, steps, warmup, want_prof=False, want_
     return res
 
 
+DUMP_ROWS = 32768                    # entity rows kept per entity-indexed array: ~33 MB at the default widths
+DUMP_LIMIT = 64 * 2 ** 20
+
+
+def dump_outputs(runner, out_dir):
+    """Writes what the runner's last step returned to its caller -- out_entity, out_relation, mask, the loss and the
+    gradient of every parameter -- as out_dir/<name>.npy in float32 (float64 for float64 tensors). Arrays indexed by entity
+    are cut to the same fixed, seeded sample of DUMP_ROWS rows, stored as `sample_rows`."""
+    import numpy as np
+    out = dict(runner.outputs)
+    for name, prm in runner.model.named_parameters():
+        if prm.grad is not None:
+            out["grad." + name] = prm.grad
+    n = runner.n
+    rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    arrays = {"sample_rows": rows.double()}
+    rows = rows.to(runner.dev)
+    for k, v in out.items():
+        v = v.detach()
+        if k in ("out_entity", "mask", "grad.entity_embeddings"):
+            v = v.index_select(0, rows)
+        arrays[k] = v.cpu().to(torch.float64 if v.dtype == torch.float64 else torch.float32)
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"output dump of {total} bytes exceeds {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a.numpy())
+    return {"dir": out_dir, "arrays": len(arrays), "bytes": total}
+
+
 def config_of(workload, world):
     """`config` of the JSON line; the reference arm prints the same object (it runs a bounded sample of this workload)."""
     return {"workload": describe(workload),
@@ -291,9 +331,15 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the secondary strong-scaling shapes (c4h, c4)")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--sub", action="store_true", help="(internal) secondary measurement in a child process")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (one GPU, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs is not None and (world > 1 or args.gpus > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs the single-GPU path (--gpus 1, --impl ours)")
     # Primary line: the C2 shape per GPU (BASELINE configs[1] at N=1; N GPUs run N x 2M entities / N x 20M edges, row-
     # partitioned: weak scaling, so the driver's per-N efficiency is well defined). Secondary keys carry BASELINE
     # configs[3] (C4, 400M edges; N >= 4) and its half c4h (fits one GPU) as STRONG-scaling measurements at every N.
@@ -304,7 +350,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        base = cpu_reference_arm(max(1, min(args.steps, 5)), max(1, min(args.warmup, 2)))
+        base = cpu_reference_arm(args.steps, args.warmup)
         line = {"impl": "reference", "metric": "SpKBGAT fwd+bwd edges/sec", "value": base["value"], "unit": "edges/s",
                 "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": base["ms_per_step"],
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -328,7 +374,9 @@ def main():
         return
 
     res = run_config(workload, world, rank, dev, args.steps, args.warmup, want_prof=True, want_e2e=not args.no_e2e,
-                     clocks=True)
+                     clocks=True, dump_dir=args.dump_outputs)
+    if "dump" in res:
+        print("[bench] outputs of the last timed step: " + json.dumps(res["dump"]), file=sys.stderr, flush=True)
     ms, e_total = res["ms"], res["e_total"]
     line = None
     if rank == 0:
@@ -430,18 +478,23 @@ class SingleGPU:
         self.graph = self.model.prepare_graph((self.edge, self.etype), self.nhop)
         self.e = edge.shape[1] + nhop.shape[0]
         self.e1, self.e2 = edge.shape[1], nhop.shape[0]
+        self.keep_outputs, self.outputs = False, None
 
     def step(self, graph=None, adj=None, nhop=None):
-        """graph: prebuilt layouts (device-timed `value`); adj / nhop: the reference's call with HOST edge tensors (`e2e`)."""
+        """graph: prebuilt layouts (device-timed `value`); adj / nhop: the reference's call with HOST edge tensors (`e2e`).
+        With `keep_outputs` set, what the step returns to its caller stays in `outputs` (the gradients stay in the model)."""
         self.model.zero_grad(set_to_none=True)
         if adj is not None:
-            out_e, out_r, _ = self.model(None, self.batch, adj, nhop)
+            out_e, out_r, mask = self.model(None, self.batch, adj, nhop)
         else:
-            out_e, out_r, _ = self.model(None, self.batch, graph or self.graph, None)
+            out_e, out_r, mask = self.model(None, self.batch, graph or self.graph, None)
         # <out_entity, G_e> + <out_relation, G_r>  (SURVEY.md 8d) as two dot products
         # (the library's deterministic reduction for the value; the backward is seeded with G_e / G_r, which is d loss / d out)
         from recon_b200 import functional as SF
-        return SF.linear_loss_backward((out_e, out_r), (self.g_ent, self.g_rel))
+        loss = SF.linear_loss_backward((out_e, out_r), (self.g_ent, self.g_rel))
+        if self.keep_outputs:
+            self.outputs = {"out_entity": out_e.detach(), "out_relation": out_r.detach(), "mask": mask, "loss": loss}
+        return loss
 
     @property
     def host(self):
