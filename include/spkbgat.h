@@ -425,6 +425,31 @@ int spk_tanh_bwd(const float* y, int64_t ldy, const float* dout, int64_t ldo, in
 int spk_rank_scores(const float* U, int64_t ldu, const float* Bt, int64_t ldb, const float* w2, const float* b2, float slope,
                     int64_t n_pairs, int32_t n_rel, int32_t D, float* out, int64_t ldo, spk_stream_t stream);
 
+/* ---- ConvKB link-prediction evaluation: filtered entity ranks (Corpus.get_validation_pred, GAT/create_batch.py:905-1199) --
+ * AC [N, 2D] (row stride ldac >= 2D) = [A | C] = E . [W1a^T | W1c^T], Bt [R, D] = Rel . W1b^T, b1 / w2 = fc1.bias / fc2.weight
+ * (fc2.bias is dropped: it shifts every score of a row alike). side 0 ranks heads: candidates (c, r, t), pair vector
+ * v_i = C[t_i] + Bt[r_i] + b1, candidate rows A[c]; side 1 ranks tails: (h, r, c), v_i = A[h_i] + Bt[r_i] + b1, rows C[c].
+ * s_c = sum_{d=0..D-1} w2[d] * lrelu(X[c,d] + v_i[d]) as one sequential fp32 chain in every kernel (so a score is the same
+ * float wherever it is computed); 1 <= D <= 512, 0 <= slope <= 1. a > b below means a > b or (isnan(a) && !isnan(b)).
+ * spk_linkpred_count:  for the test triples int64 [T,3] (h, r, t) writes V [T, ldv >= D] = v_i, true_id int32 [T] = the
+ *                      ranked entity (-1 when keep[i] == 0 or an id is out of range; keep uint8 [T] may be null = keep all),
+ *                      s_true float [T] and count int32 [T] = #{c in [0,N), c != true_id[i] : s_c > s_true[i]}; the
+ *                      T x N scores are never stored. An id outside [0, N) / [0, R) sets bit 0 of *err_flag.
+ * spk_linkpred_filter: after spk_linkpred_count on the same arguments and stream: keys int64 [n_keys] are the sorted,
+ *                      possibly repeated spk_triple_keys of the known triples, in (h, r, t) order for side 1 and of the
+ *                      column-swapped (t, r, h) triples for side 0, so row i's known candidates are one key range;
+ *                      subtracts from count[i] each distinct known candidate c != true_id[i] with s_c > s_true[i].
+ *                      work: int64 [3T + 1] scratch. A decoded id outside [0, N) sets bit 1 of *err_flag.
+ * The filtered rank of row i is 1 + count[i] (the position of the test triple under a stable descending sort). */
+int spk_linkpred_count(const float* AC, int64_t ldac, int64_t n_ent, const float* Bt, int64_t ldb, int64_t n_rel,
+                       const float* b1, const float* w2, float slope, int32_t D, const int64_t* triples,
+                       const uint8_t* keep, int64_t n_pairs, int32_t side, float* V, int64_t ldv, float* s_true,
+                       int32_t* true_id, int32_t* count, int32_t* err_flag, spk_stream_t stream);
+int spk_linkpred_filter(const float* AC, int64_t ldac, int64_t n_ent, int64_t n_rel, const float* w2, float slope,
+                        int32_t D, const int64_t* triples, int64_t n_pairs, int32_t side, const float* V, int64_t ldv,
+                        const float* s_true, const int32_t* true_id, const int64_t* keys, int64_t n_keys, int64_t* work,
+                        int32_t* count, int32_t* err_flag, spk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

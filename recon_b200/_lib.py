@@ -214,6 +214,10 @@ SIGNATURES = {
     "spk_tanh_fwd": (_I32, [_VP, _I64, _I64, _I32, _VP]),
     "spk_tanh_bwd": (_I32, [_VP, _I64, _VP, _I64, _I64, _I32, _VP, _I64, _VP]),
     "spk_rank_scores": (_I32, [_VP, _I64, _VP, _I64, _VP, _VP, C.c_float, _I64, _I32, _I32, _VP, _I64, _VP]),
+    "spk_linkpred_count": (_I32, [_VP, _I64, _I64, _VP, _I64, _I64, _VP, _VP, C.c_float, _I32, _VP, _VP, _I64, _I32,
+                                  _VP, _I64, _VP, _VP, _VP, _VP, _VP]),
+    "spk_linkpred_filter": (_I32, [_VP, _I64, _I64, _I64, _VP, C.c_float, _I32, _VP, _I64, _I32, _VP, _I64, _VP, _VP,
+                                   _VP, _I64, _VP, _VP, _VP, _VP]),
     "spk_export_json": (_I32, [_VP, _I64, _I64, _I64, C.c_char_p, _I32]),
     "spk_export_bin": (_I32, [_VP, _I64, _I64, _I64, C.c_char_p]),
     "spk_import_json_shape": (_I32, [C.c_char_p, C.POINTER(_I64), C.POINTER(_I64)]),
