@@ -92,7 +92,8 @@ int64_t spk_gemm_tc_workspace_floats(int32_t N, int32_t K);
 int spk_gemm_nn_tc(const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
                    int64_t M, int32_t N, int32_t K, int32_t accumulate, float* workspace, spk_stream_t stream);
 
-/* Same, with an epilogue on the final value: act = 0 none, 1 = ELU (F.elu at GAT/layers.py:175 / models.py:86). */
+/* Same, with an epilogue on the final value: act = 0 none, 1 = ELU (F.elu at GAT/layers.py:175 / models.py:86),
+ * 2 = tanh (GAT_sep_space/models.py:316-320; the tanhf of spk_tanh_fwd, bit-equal to the product followed by it). */
 int spk_gemm_nn_tc_act(const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
                        int64_t M, int32_t N, int32_t K, int32_t accumulate, int32_t act, float* workspace,
                        spk_stream_t stream);

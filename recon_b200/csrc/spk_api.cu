@@ -150,7 +150,7 @@ int spk_gemm_nn_tc_act(const float* A, int64_t lda, const float* B, int64_t ldb,
     if (lda < K || ldb < N || ldc < N) { set_error("gemm_nn_tc_act: leading dimension too small"); return 1; }
     if (!gemm_nn_tc_supported(A, lda, M, N, K)) { set_error("gemm_nn_tc_act: A must be 16-byte aligned with lda %% 4 == 0"); return 1; }
     if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 15)) { set_error("gemm_nn_tc_act: aligned workspace required"); return 1; }
-    if (act < 0 || act > 1) { set_error("gemm_nn_tc_act: unknown activation %d", act); return 1; }
+    if (act < 0 || act > 2) { set_error("gemm_nn_tc_act: unknown activation %d", act); return 1; }
     return gemm_nn_tc(A, lda, B, ldb, C, ldc, M, N, K, accumulate, workspace, (cudaStream_t)stream, act);
 }
 int spk_elu_inplace(float* x, int64_t ldx, int64_t n_rows, int32_t width, spk_stream_t stream) {

@@ -98,7 +98,8 @@ __device__ __forceinline__ uint64_t make_kmajor_sw128_desc(uint32_t saddr) {
 
 struct TcParams {
     float* C; long ldc; long M; int N; int K; int BN; int n_tiles_n; int stages; int accumulate; int c_vec;
-    int act;                                    // epilogue: 0 = none, 1 = ELU (GAT/layers.py:175) on the final value
+    int act;                                    // epilogue on the final value: 0 = none, 1 = ELU (GAT/layers.py:175),
+                                                // 2 = tanh (GAT_sep_space/models.py:316-320)
     int c_tma;                                  // epilogue stores through shared memory + TMA (coalesced 128 B rows)
     int raw_hi;                                 // the MMA reads the raw fp32 tile as "hi" (kind::tf32 ignores the low 13 mantissa bits)
     int cs;                                     // cluster size (1 or 2): the CTAs of a cluster work on consecutive M tiles of the
@@ -112,6 +113,10 @@ __device__ __forceinline__ float tc_elu(float x) {
     const float neg = x > -0.125f ? small : big;
     return x > 0.f ? x : neg;
 }
+
+// The epilogue activation of act != 0 (the TMA-store epilogues branch once per chunk instead); tanh is the libdevice tanhf
+// of tanh_fwd_kernel (spk_convkb.cu, no fast-math), so act = 2 gives the same bits as the product followed by spk_tanh_fwd.
+__device__ __forceinline__ float tc_act(float x, int act) { return act == 2 ? tanhf(x) : tc_elu(x); }
 
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmBhi,
@@ -275,7 +280,10 @@ gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                       "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
                     : "r"(taddr));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (p.act) {
+                if (p.act == 2) {
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(tanhf(__uint_as_float(r[j])));
+                } else if (p.act) {
 #pragma unroll
                     for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(tc_elu(__uint_as_float(r[j])));
                 }
@@ -335,7 +343,7 @@ gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                         float4 o = make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]), __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3]));
                         if (p.c_vec && col + 3 < p.N) {
                             if (p.accumulate) o = f4add(o, *reinterpret_cast<const float4*>(crow + col));
-                            if (p.act) o = make_float4(tc_elu(o.x), tc_elu(o.y), tc_elu(o.z), tc_elu(o.w));
+                            if (p.act) o = make_float4(tc_act(o.x, p.act), tc_act(o.y, p.act), tc_act(o.z, p.act), tc_act(o.w, p.act));
                             *reinterpret_cast<float4*>(crow + col) = o;
                         } else {
                             const float ov[4] = {o.x, o.y, o.z, o.w};
@@ -343,7 +351,7 @@ gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                             for (int k = 0; k < 4; ++k)
                                 if (col + k < p.N) {
                                     const float r1 = p.accumulate ? crow[col + k] + ov[k] : ov[k];
-                                    crow[col + k] = p.act ? tc_elu(r1) : r1;
+                                    crow[col + k] = p.act ? tc_act(r1, p.act) : r1;
                                 }
                         }
                     }
@@ -552,7 +560,10 @@ gemm_nn_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                       "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
                     : "r"(taddr));
                 asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                if (p.act) {
+                if (p.act == 2) {
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(tanhf(__uint_as_float(r[j])));
+                } else if (p.act) {
 #pragma unroll
                     for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(tc_elu(__uint_as_float(r[j])));
                 }

@@ -19,7 +19,14 @@ namespace spk {
 namespace {
 
 constexpr int LP_MAX_D = 512;
-constexpr int LP_BP = 128, LP_BC = 128, LP_BK = 8;       // pairs x candidates per CTA tile, k-chunk per pipeline stage
+constexpr int LP_BC = 128, LP_BK = 8;                    // candidates per CTA tile, k-chunk per pipeline stage
+// Pair-tile heights of lp_count_kernel: a call with at most LP_NARROW_MAX pairs uses LP_BP_NARROW-row tiles, so a small
+// test set (one relation group of the GAT_sep_space evaluation, usually 1-3 rows) does not pay for 128 padded pairs
+// against all N candidates; larger calls use 128-row tiles, which reuse every staged candidate value 8x more often.
+// Crossover measured with profiles/bench_linkpred_sep.py on a B200 (DESIGN.md section 9, N4b): n pairs as 16-row tiles
+// cost 1.41 ms per 16 rows at N = 2M, D = 200, one 128-row tile 8.04 ms: 7.04 ms at 80 pairs, 8.44 ms at 96.
+constexpr int LP_BP_WIDE = 128, LP_BP_NARROW = 16;
+constexpr long LP_NARROW_MAX = 80;
 
 __device__ __forceinline__ float lp_step(float acc, float x_c, float v, float w, float slope) {
     const float x = __fadd_rn(x_c, v);
@@ -62,33 +69,45 @@ lp_pairs_kernel(const float* __restrict__ AC, long ldac, long N, const float* __
     }
 }
 
+// Pair row of micro-tile row i of thread row ty in a BP-row tile: 128 rows: ty*4 + {0..3}, 64 + ty*4 + {0..3};
+// narrower tiles: ty*(BP/16) + i.
+template <int BP>
+__device__ __forceinline__ int lp_pair_row(int i, int ty) {
+    if constexpr (BP == 128) return i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4);
+    else return ty * (BP / 16) + i;
+}
+
 // count[i] += #{c : c != true_i, s_c > s_true_i} for the candidate tiles blockIdx.y, blockIdx.y + gridDim.y, ...
-// CTA tile: 128 pairs x 128 candidates, 16 x 16 threads with an 8 x 8 register micro-tile each (rows ty*4 + {0..3},
-// 64 + ty*4 + {0..3}; columns likewise with tx). V and X chunks of 8 k are staged through registers into double-buffered,
+// CTA tile: BP pairs x 128 candidates, 16 x 16 threads with a BP/16 x 8 register micro-tile each (rows lp_pair_row,
+// columns tx*4 + {0..3}, 64 + tx*4 + {0..3}). V and X chunks of 8 k are staged through registers into double-buffered,
 // transposed shared memory (the spk_gemm_simt.cu pipeline, carried across candidate tiles). After the last k chunk of a
-// tile each thread compares its 64 finished scores and counts in registers; the 16 threads of a pair row are summed by
-// shuffles and added with one integer atomic per pair and CTA (order-independent, so counts are reproducible).
+// tile each thread compares its finished scores and counts in registers; the 16 threads of a pair row are summed by
+// shuffles and added with one integer atomic per pair and CTA (order-independent, so counts are reproducible). Every
+// score is the same lp_step chain whatever BP is, so every tile height gives the same counts.
+template <int BP>
 __global__ void __launch_bounds__(256, 2)
 lp_count_kernel(const float* __restrict__ X, long ldx, long N, const float* __restrict__ V, long ldv,
                 const float* __restrict__ w2, float slope, int D, const float* __restrict__ s_true,
                 const int* __restrict__ true_id, long T, int x_vec, int v_vec, int* __restrict__ count) {
-    __shared__ __align__(16) float Vs[2][LP_BK][LP_BP + 4];
+    static_assert(BP == 128 || (BP % 16 == 0 && BP / 16 <= 4), "pair tile: 128 rows, or 16 * (1..4)");
+    constexpr int MI = BP / 16;                                   // micro-tile rows per thread
+    __shared__ __align__(16) float Vs[2][LP_BK][BP + 4];
     __shared__ __align__(16) float Xs[2][LP_BK][LP_BC + 4];
     __shared__ float w2s[LP_MAX_D + LP_BK];
     const int tid = threadIdx.x;
     const int tx = tid & 15, ty = tid >> 4;
-    const long p0 = (long)blockIdx.x * LP_BP;
+    const long p0 = (long)blockIdx.x * BP;
 
     int live = 0;
-    for (int k = tid; k < LP_BP; k += 256) live |= (p0 + k < T && true_id[p0 + k] >= 0);
+    for (int k = tid; k < BP; k += 256) live |= (p0 + k < T && true_id[p0 + k] >= 0);
     if (!__syncthreads_or(live)) return;                          // every row of this tile is skipped
     for (int d = tid; d < LP_MAX_D + LP_BK; d += 256) w2s[d] = d < D ? __ldg(w2 + d) : 0.f;
 
-    float st[8];
-    int tr[8], cnt[8];
+    float st[MI];
+    int tr[MI], cnt[MI];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        const long p = p0 + (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
+    for (int i = 0; i < MI; ++i) {
+        const long p = p0 + lp_pair_row<BP>(i, ty);
         tr[i] = p < T ? true_id[p] : -1;
         st[i] = p < T ? s_true[p] : 0.f;
         cnt[i] = 0;
@@ -114,24 +133,29 @@ lp_count_kernel(const float* __restrict__ X, long ldx, long N, const float* __re
 #pragma unroll
             for (int e = 0; e < 4; ++e) rx[e] = (c < N && k + e < D) ? __ldg(X + c * ldx + k + e) : 0.f;
         }
-        if (p < T && v_vec && k + 3 < D) {
-            const float4 q = ldg4(V + p * ldv + k);
-            rv[0] = q.x; rv[1] = q.y; rv[2] = q.z; rv[3] = q.w;
-        } else {
+        if (BP == 128 || l_row < BP) {                             // the V tile has BP rows
+            if (p < T && v_vec && k + 3 < D) {
+                const float4 q = ldg4(V + p * ldv + k);
+                rv[0] = q.x; rv[1] = q.y; rv[2] = q.z; rv[3] = q.w;
+            } else {
 #pragma unroll
-            for (int e = 0; e < 4; ++e) rv[e] = (p < T && k + e < D) ? __ldg(V + p * ldv + k + e) : 0.f;
+                for (int e = 0; e < 4; ++e) rv[e] = (p < T && k + e < D) ? __ldg(V + p * ldv + k + e) : 0.f;
+            }
         }
         ld_k += LP_BK;
         if (ld_k >= D) { ld_k = 0; ld_c += c_step; }
     };
     auto store = [&](int buf) {
 #pragma unroll
-        for (int e = 0; e < 4; ++e) { Xs[buf][l_k + e][l_row] = rx[e]; Vs[buf][l_k + e][l_row] = rv[e]; }
+        for (int e = 0; e < 4; ++e) {
+            Xs[buf][l_k + e][l_row] = rx[e];
+            if (BP == 128 || l_row < BP) Vs[buf][l_k + e][l_row] = rv[e];
+        }
     };
 
-    float acc[8][8];
+    float acc[MI][8];
 #pragma unroll
-    for (int i = 0; i < 8; ++i)
+    for (int i = 0; i < MI; ++i)
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
 
@@ -147,14 +171,21 @@ lp_count_kernel(const float* __restrict__ X, long ldx, long N, const float* __re
         for (int k = 0; k < LP_BK; ++k) {
             if (k < kn) {
                 const float w = w2s[k0 + k];
-                const float4 v0 = *reinterpret_cast<const float4*>(&Vs[buf][k][ty * 4]);
-                const float4 v1 = *reinterpret_cast<const float4*>(&Vs[buf][k][64 + ty * 4]);
+                float vv[MI];
+                if constexpr (BP == 128) {
+                    const float4 v0 = *reinterpret_cast<const float4*>(&Vs[buf][k][ty * 4]);
+                    const float4 v1 = *reinterpret_cast<const float4*>(&Vs[buf][k][64 + ty * 4]);
+                    vv[0] = v0.x; vv[1] = v0.y; vv[2] = v0.z; vv[3] = v0.w;
+                    vv[4] = v1.x; vv[5] = v1.y; vv[6] = v1.z; vv[7] = v1.w;
+                } else {
+#pragma unroll
+                    for (int i = 0; i < MI; ++i) vv[i] = Vs[buf][k][ty * MI + i];
+                }
                 const float4 x0 = *reinterpret_cast<const float4*>(&Xs[buf][k][tx * 4]);
                 const float4 x1 = *reinterpret_cast<const float4*>(&Xs[buf][k][64 + tx * 4]);
-                const float vv[8] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w};
                 const float xv[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
 #pragma unroll
-                for (int i = 0; i < 8; ++i)
+                for (int i = 0; i < MI; ++i)
 #pragma unroll
                     for (int j = 0; j < 8; ++j) acc[i][j] = lp_step(acc[i][j], xv[j], vv[i], w, slope);
             }
@@ -166,7 +197,7 @@ lp_count_kernel(const float* __restrict__ X, long ldx, long N, const float* __re
                 const long c = c0 + (j < 4 ? tx * 4 + j : 64 + tx * 4 + (j - 4));
                 const bool cv = c < N;
 #pragma unroll
-                for (int i = 0; i < 8; ++i) {
+                for (int i = 0; i < MI; ++i) {
                     cnt[i] += (cv && c != tr[i] && lp_gt(acc[i][j], st[i])) ? 1 : 0;
                     acc[i][j] = 0.f;
                 }
@@ -180,11 +211,11 @@ lp_count_kernel(const float* __restrict__ X, long ldx, long N, const float* __re
         }
     }
 #pragma unroll
-    for (int i = 0; i < 8; ++i) {
+    for (int i = 0; i < MI; ++i) {
         int c = cnt[i];
 #pragma unroll
         for (int o = 1; o < 16; o <<= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-        const long p = p0 + (i < 4 ? ty * 4 + i : 64 + ty * 4 + (i - 4));
+        const long p = p0 + lp_pair_row<BP>(i, ty);
         if (tx == 0 && tr[i] >= 0 && c) atomicAdd(count + p, c);   // tr[i] >= 0 implies p < T
     }
 }
@@ -287,6 +318,26 @@ lp_discount_kernel(const float* __restrict__ X, long ldx, long long N, long long
     }
 }
 
+template <int BP>
+int lp_launch_count(const float* X, long ldac, long n_ent, const float* V, long ldv, const float* w2, float slope, int D,
+                    const float* s_true, const int* true_id, long n_pairs, int x_vec, int v_vec, int* count, cudaStream_t s) {
+    int dev = 0, sms = 148, occ = 1;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lp_count_kernel<BP>, 256, 0);
+    const long gx = (n_pairs + BP - 1) / BP;
+    const long n_ct = (n_ent + LP_BC - 1) / LP_BC;
+    // one resident wave when the pair tiles allow it; the CTAs of one blockIdx.y walk the same candidate tiles together,
+    // so each candidate row comes from HBM about once and from L2 for the other pair tiles
+    long gy = (long)sms * (occ > 0 ? occ : 1) / gx;
+    gy = gy < 1 ? 1 : (gy > n_ct ? n_ct : gy);
+    if (gy > 65535) gy = 65535;
+    if (gx > 0x7fffffffL) { set_error("linkpred_count: too many test rows"); return 1; }
+    lp_count_kernel<BP><<<dim3((unsigned)gx, (unsigned)gy), 256, 0, s>>>(X, ldac, n_ent, V, ldv, w2, slope, D, s_true,
+                                                                        true_id, n_pairs, x_vec, v_vec, count);
+    return check_launch("linkpred_count");
+}
+
 int lp_check(const char* who, long long ldac, long long n_ent, long long n_rel, float slope, int D, int side) {
     if (D < 1 || ldac < 2LL * D || n_ent < 1 || n_ent >= (1LL << 31) - 1 || n_rel < 1 || (side != 0 && side != 1)) {
         set_error("%s: bad arguments", who);
@@ -321,21 +372,10 @@ int spk_linkpred_count(const float* AC, int64_t ldac, int64_t n_ent, const float
     const float* X = AC + (side ? D : 0);
     const int x_vec = (ldac % 4 == 0) && ((reinterpret_cast<uintptr_t>(X) & 15) == 0);
     const int v_vec = (ldv % 4 == 0) && ((reinterpret_cast<uintptr_t>(V) & 15) == 0);
-    int dev = 0, sms = 148, occ = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lp_count_kernel, 256, 0);
-    const long gx = (n_pairs + LP_BP - 1) / LP_BP;
-    const long n_ct = (n_ent + LP_BC - 1) / LP_BC;
-    // one resident wave when the pair tiles allow it; the CTAs of one blockIdx.y walk the same candidate tiles together,
-    // so each candidate row comes from HBM about once and from L2 for the other pair tiles
-    long gy = (long)sms * (occ > 0 ? occ : 1) / gx;
-    gy = gy < 1 ? 1 : (gy > n_ct ? n_ct : gy);
-    if (gy > 65535) gy = 65535;
-    if (gx > 0x7fffffffL) { set_error("linkpred_count: too many test rows"); return 1; }
-    lp_count_kernel<<<dim3((unsigned)gx, (unsigned)gy), 256, 0, s>>>(X, (long)ldac, (long)n_ent, V, (long)ldv, w2, slope, D,
-                                                                    s_true, true_id, (long)n_pairs, x_vec, v_vec, count);
-    return check_launch("linkpred_count");
+    if (n_pairs <= LP_NARROW_MAX)
+        return lp_launch_count<LP_BP_NARROW>(X, ldac, n_ent, V, ldv, w2, slope, D, s_true, true_id, n_pairs, x_vec, v_vec,
+                                             count, s);
+    return lp_launch_count<LP_BP_WIDE>(X, ldac, n_ent, V, ldv, w2, slope, D, s_true, true_id, n_pairs, x_vec, v_vec, count, s);
 }
 
 int spk_linkpred_filter(const float* AC, int64_t ldac, int64_t n_ent, int64_t n_rel, const float* w2, float slope,

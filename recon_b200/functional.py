@@ -139,7 +139,7 @@ def _extended_weights_torch(a_list, a2_list, in_features, geom):
 
 def gemm_nn(A, B, out=None, accumulate=False, act=0):
     """out[M,N] (+)= A[M,K] @ B[K,N] on the library's GEMM (row-major, last-dim contiguous views allowed).
-    act=1 applies ELU to the final value (fused into the tensor-core epilogue)."""
+    act=1 applies ELU, act=2 tanh to the final value (fused into the tensor-core epilogue)."""
     assert A.dim() == 2 and B.dim() == 2 and A.shape[1] == B.shape[0]
     assert A.stride(1) == 1 and B.stride(1) == 1
     M, K = A.shape
@@ -166,7 +166,9 @@ def gemm_nn(A, B, out=None, accumulate=False, act=0):
         else:
             _lib.check(lib.spk_gemm_nn(_lib.ptr(A), A.stride(0), _lib.ptr(B), B.stride(0), _lib.ptr(out),
                                        out.stride(0), M, N, K, int(accumulate), _lib.stream_ptr()), "gemm_nn")
-        if act:
+        if act == 2:
+            _lib.check(lib.spk_tanh_fwd(_lib.ptr(out), out.stride(0), M, N, _lib.stream_ptr()), "tanh_fwd")
+        elif act:
             _lib.check(lib.spk_elu_inplace(_lib.ptr(out), out.stride(0), M, N, _lib.stream_ptr()), "elu_inplace")
     return out
 
