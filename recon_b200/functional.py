@@ -137,10 +137,19 @@ def _extended_weights_torch(a_list, a2_list, in_features, geom):
 
 # ---- dense products --------------------------------------------------------------------------
 
+def _unit_col_stride(T):
+    """A one-column matrix counts as contiguous whatever its column stride (W.t().contiguous() of a one-row W keeps
+    the row length there); the kernels address it through the row stride alone, so give it column stride 1."""
+    if T is not None and T.stride(1) != 1 and T.shape[1] == 1:
+        return T.as_strided(T.shape, (T.stride(0), 1))
+    return T
+
+
 def gemm_nn(A, B, out=None, accumulate=False, act=0):
     """out[M,N] (+)= A[M,K] @ B[K,N] on the library's GEMM (row-major, last-dim contiguous views allowed).
     act=1 applies ELU, act=2 tanh to the final value (fused into the tensor-core epilogue)."""
     assert A.dim() == 2 and B.dim() == 2 and A.shape[1] == B.shape[0]
+    A, B, out = _unit_col_stride(A), _unit_col_stride(B), _unit_col_stride(out)
     assert A.stride(1) == 1 and B.stride(1) == 1
     M, K = A.shape
     N = B.shape[1]
@@ -176,6 +185,7 @@ def gemm_nn(A, B, out=None, accumulate=False, act=0):
 def gemm_tn(A, B, out=None, accumulate=False):
     """out[Ka,Nb] (+)= A[M,Ka]^T @ B[M,Nb], deterministic fixed-order split over M."""
     assert A.dim() == 2 and B.dim() == 2 and A.shape[0] == B.shape[0]
+    A, B, out = _unit_col_stride(A), _unit_col_stride(B), _unit_col_stride(out)
     assert A.stride(1) == 1 and B.stride(1) == 1
     M, Ka = A.shape
     Nb = B.shape[1]
