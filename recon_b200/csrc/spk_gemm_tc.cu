@@ -700,7 +700,9 @@ int gemm_nn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
     const int b_tile = BN * 128;
     const int stage_bytes = 2 * TC_A_TILE + 2 * b_tile;
     const int c_vec = (ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
-    const int c_tma = c_vec && !(act && accumulate);
+    // the TMA epilogue writes a row's last box up to the next 16-byte boundary: with N % 4 != 0 it reaches the floats past
+    // column N, outside the caller's view (seen on a B200: C += put NaN there in rows whose product is NaN)
+    const int c_tma = c_vec && (N % 4 == 0) && !(act && accumulate);
     const int staging = c_tma ? 4 * 8192 : 0;                       // 4 epilogue warps x 2 x [32 x 32] fp32
     int stages = (225 * 1024 - 1024 - staging) / stage_bytes;
     if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
