@@ -451,6 +451,53 @@ int spk_linkpred_filter(const float* AC, int64_t ldac, int64_t n_ent, int64_t n_
                         const float* s_true, const int32_t* true_id, const int64_t* keys, int64_t n_keys, int64_t* work,
                         int32_t* count, int32_t* err_flag, spk_stream_t stream);
 
+/* ---- GAT_sep_space relation-space projection: tanh(e . W_ent2rel[r]) per row, grouped by relation on the device ----
+ * Reference: GAT_sep_space/models.py:316-320 and the TransE loss of GAT_sep_space/main.py:360-377. No call reads a
+ * device value back: buffers are sized for the worst case, G_max = min(n_rel, n_rows) groups and
+ * M_max = 128 * ceil((n_rows + 127 * G_max) / 128) padded rows.
+ * spk_ent2rel_keys:      rows j < reps * n_src: key[j] = rel[(j % n_src) * stride] or n_rel when that id is outside
+ *                        [0, n_rel) (sets *err_flag; such a row joins no group), val[j] = j. Sort with spk_sort_pairs and
+ *                        take segptr = spk_segment_ptr(keys, n_rel).
+ * spk_ent2rel_plan:      one launch; groups = relations present, ascending. Group g owns the 128-row M tiles
+ *                        [group_tile0[g], group_tile0[g+1]) (its rows in sorted order, then zero pad rows) and the
+ *                        weight-gradient tasks [task_ptr[g], task_ptr[g+1]) of tiles_per_task tiles each, task z covering
+ *                        real rows [task_row0[z], task_row1[z]); rel2group[r] = g or -1; tile_group[t] = g;
+ *                        counts[3] = {groups, M tiles, tasks}. Sizes: rel2group n_rel, group_rel G_max, group_tile0 and
+ *                        task_ptr G_max + 1, tile_group M_max / 128, task_row0 / task_row1 the task bound.
+ * spk_ent2rel_positions: pos int64 [n_rows] = padded row of every input row (0 for a row without group).
+ * spk_ent2rel_gather:    out[p, :width] = table[ids ? ids[src] : src] for the real padded rows (src = their input row),
+ *                        zero for pad rows; rows past counts[1] * 128 are not written. An id outside [0, n_table) sets
+ *                        *err_flag and writes a zero row.
+ * spk_gemm_nn_tc_grouped: C_g = act(A_g . B_g) over the M tiles of every group (3xTF32 tcgen05, act 0 or 2 = tanh),
+ *                        B_g[k, n] = W[group_rel[g] * rstride + n * sn + k * sk]: sn = 1, sk = N is W[r] ([K, N]
+ *                        row-major), sn = ld, sk = 1 its transpose. Bit-identical per group to spk_gemm_nn_tc_act on that
+ *                        group's rows alone. workspace: spk_gemm_nn_tc_grouped_workspace_floats(G_max, N, K).
+ * spk_gemm_tn_tc_grouped: C[r] ([Ka, Nb] contiguous, for every r < n_rel) = sum over the tasks of group rel2group[r], in
+ *                        task order, of A[rows]^T B[rows]; zero for relations without rows. No atomics.
+ *                        workspace: spk_gemm_tn_tc_grouped_workspace_floats(max_tasks, Ka, Nb). */
+int spk_ent2rel_keys(const int64_t* rel, int64_t stride, int64_t n_src, int32_t reps, int32_t n_rel, int32_t* keys,
+                     int32_t* vals, int32_t* err_flag, spk_stream_t stream);
+int spk_ent2rel_plan(const int32_t* segptr, int32_t n_rel, int32_t tiles_per_task, int32_t* rel2group,
+                     int32_t* group_rel, int32_t* group_tile0, int32_t* task_ptr, int32_t* tile_group,
+                     int32_t* task_row0, int32_t* task_row1, int32_t* counts, spk_stream_t stream);
+int spk_ent2rel_positions(const int32_t* sorted_keys, const int32_t* sorted_vals, int64_t n_rows, int32_t n_rel,
+                          const int32_t* segptr, const int32_t* rel2group, const int32_t* group_tile0, int64_t* pos,
+                          spk_stream_t stream);
+int spk_ent2rel_gather(const float* table, int64_t ldt, int64_t n_table, const int64_t* ids, const int32_t* sorted_vals,
+                       const int32_t* segptr, const int32_t* group_rel, const int32_t* group_tile0,
+                       const int32_t* tile_group, const int32_t* counts, int32_t width, int64_t max_rows, float* out,
+                       int64_t ldo, int32_t* err_flag, spk_stream_t stream);
+int64_t spk_gemm_nn_tc_grouped_workspace_floats(int32_t max_groups, int32_t N, int32_t K);
+int spk_gemm_nn_tc_grouped(const float* A, int64_t lda, int64_t max_rows, const float* W, int64_t rstride, int64_t sn,
+                           int64_t sk, int32_t N, int32_t K, const int32_t* group_rel, const int32_t* counts,
+                           int32_t max_groups, const int32_t* tile_group, float* C, int64_t ldc, int32_t act,
+                           float* workspace, spk_stream_t stream);
+int64_t spk_gemm_tn_tc_grouped_workspace_floats(int32_t max_tasks, int32_t Ka, int32_t Nb);
+int spk_gemm_tn_tc_grouped(const float* A, int64_t lda, const float* B, int64_t ldb, int64_t max_rows, int32_t Ka,
+                           int32_t Nb, const int32_t* task_row0, const int32_t* task_row1, const int32_t* counts,
+                           int32_t max_tasks, const int32_t* rel2group, const int32_t* task_ptr, int32_t n_rel, float* C,
+                           float* workspace, spk_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -218,6 +218,16 @@ SIGNATURES = {
                                   _VP, _I64, _VP, _VP, _VP, _VP, _VP]),
     "spk_linkpred_filter": (_I32, [_VP, _I64, _I64, _I64, _VP, C.c_float, _I32, _VP, _I64, _I32, _VP, _I64, _VP, _VP,
                                    _VP, _I64, _VP, _VP, _VP, _VP]),
+    "spk_ent2rel_keys": (_I32, [_VP, _I64, _I64, _I32, _I32, _VP, _VP, _VP, _VP]),
+    "spk_ent2rel_plan": (_I32, [_VP, _I32, _I32, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "spk_ent2rel_positions": (_I32, [_VP, _VP, _I64, _I32, _VP, _VP, _VP, _VP, _VP]),
+    "spk_ent2rel_gather": (_I32, [_VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I32, _I64, _VP, _I64, _VP, _VP]),
+    "spk_gemm_nn_tc_grouped_workspace_floats": (_I64, [_I32, _I32, _I32]),
+    "spk_gemm_nn_tc_grouped": (_I32, [_VP, _I64, _I64, _VP, _I64, _I64, _I64, _I32, _I32, _VP, _VP, _I32, _VP, _VP, _I64,
+                                      _I32, _VP, _VP]),
+    "spk_gemm_tn_tc_grouped_workspace_floats": (_I64, [_I32, _I32, _I32]),
+    "spk_gemm_tn_tc_grouped": (_I32, [_VP, _I64, _VP, _I64, _I64, _I32, _I32, _VP, _VP, _VP, _I32, _VP, _VP, _I32, _VP,
+                                      _VP, _VP]),
     "spk_export_json": (_I32, [_VP, _I64, _I64, _I64, C.c_char_p, _I32]),
     "spk_export_bin": (_I32, [_VP, _I64, _I64, _I64, C.c_char_p]),
     "spk_import_json_shape": (_I32, [C.c_char_p, C.POINTER(_I64), C.POINTER(_I64)]),

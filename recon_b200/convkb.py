@@ -6,7 +6,9 @@
   SpKBGATConvOnly   <- GAT/models.py:242-304   forward(Corpus_, adj, batch_inputs) / batch_test(batch_inputs); with a
                        GAT_sep_space/models.py:311-339   `model_gat` argument the head / tail rows go through
                                                tanh(e . W_ent2rel[r]) first (relation-space projection)
-  ent2rel_project   <- GAT_sep_space/models.py:316-320, GAT_sep_space/main.py:360-377
+  ent2rel_project   <- GAT_sep_space/models.py:316-320, GAT_sep_space/main.py:360-377 (RelationLayout + GroupedProjectFn:
+                       rows grouped by relation on the device, one grouped tcgen05 GEMM per pass; also the projection of
+                       the sep-space TransE loss, loss.batch_gat_loss(..., model_gat=))
   relation_scores / rank_relations <- GAT/create_batch.py:1367-1500 (every test pair scored under every relation)
 
 fc1 over the concatenation [h | r | t] is one tcgen05 GEMM on the gathered rows for training batches (a few thousand
@@ -21,6 +23,7 @@ import torch.nn as nn
 
 from . import _lib
 from . import functional as SF
+from .graph import sort_pairs, _segment_ptr, _key_bits
 from .layers import SpecialSpmmFunctionFinal
 
 LRELU_SLOPE = 0.01          # nn.LeakyReLU() default, GAT/layers.py:25
@@ -114,53 +117,155 @@ class TanhFn(torch.autograd.Function):
         return d
 
 
-class _GroupedMatMulFn(torch.autograd.Function):
-    """Y[b] = X[b] . W[r_b] for rows sorted by relation (segments given by host offsets): one GEMM per relation
-    present; dW[r] = X_seg^T dY_seg, dX_seg = dY_seg . W[r]^T (torch.bmm of GAT_sep_space/models.py:319-320, grouped)."""
+TILES_PER_TASK = 8          # a weight-gradient task of the grouped projection: up to 8 x 128 rows of one relation
+
+
+def _ld4(d):
+    return (d + 3) // 4 * 4
+
+
+class RelationLayout:
+    """Rows grouped by relation for the grouped tensor-core projection, built on the device (spk_ent2rel_*).
+
+    Row j (j < reps * n_src) has relation rel[(j % n_src) * stride] (an int64 tensor view). Rows are stably sorted by
+    relation; every relation present is one group, padded with zero rows to whole 128-row M tiles, so no tile straddles
+    two relations. The host never reads the group count back: buffers are sized for the worst case, min(n_rel, rows)
+    groups of 127 pad rows each. `pos[j]` is row j's padded row; `err` is set for a relation id outside [0, n_rel), whose
+    row joins no group (so W_ent2rel is never read out of range) and has pos 0."""
+
+    def __init__(self, rel, n_src, reps, stride, n_rel):
+        lib = _lib.load()
+        dev = rel.device
+        n = int(n_src) * int(reps)
+        self.n_rows, self.n_rel = n, int(n_rel)
+        self.max_groups = max(1, min(self.n_rel, n))
+        self.max_tiles = (n + 127 * self.max_groups + 127) // 128
+        self.max_rows = 128 * self.max_tiles
+        self.max_tasks = min(self.max_tiles, (self.max_tiles + (TILES_PER_TASK - 1) * self.max_groups) // TILES_PER_TASK)
+        i32 = dict(dtype=torch.int32, device=dev)
+        keys, vals = torch.empty(n, **i32), torch.empty(n, **i32)
+        self.err = torch.zeros(1, **i32)
+        _lib.check(lib.spk_ent2rel_keys(rel.data_ptr(), stride, n_src, reps, self.n_rel, keys.data_ptr(), vals.data_ptr(),
+                                        self.err.data_ptr(), _lib.stream_ptr()), "ent2rel_keys")
+        self.keys, self.vals = sort_pairs(keys, vals, _key_bits(self.n_rel + 1))
+        self.segptr = _segment_ptr(self.keys, self.n_rel)
+        self.rel2group = torch.empty(self.n_rel, **i32)
+        self.group_rel = torch.empty(self.max_groups, **i32)
+        self.group_tile0 = torch.empty(self.max_groups + 1, **i32)
+        self.task_ptr = torch.empty(self.max_groups + 1, **i32)
+        self.tile_group = torch.empty(self.max_tiles, **i32)
+        self.task_row0 = torch.empty(max(1, self.max_tasks), **i32)
+        self.task_row1 = torch.empty(max(1, self.max_tasks), **i32)
+        self.counts = torch.empty(3, **i32)                      # groups, M tiles, tasks (device only)
+        _lib.check(lib.spk_ent2rel_plan(self.segptr.data_ptr(), self.n_rel, TILES_PER_TASK, self.rel2group.data_ptr(),
+                                        self.group_rel.data_ptr(), self.group_tile0.data_ptr(), self.task_ptr.data_ptr(),
+                                        self.tile_group.data_ptr(), self.task_row0.data_ptr(), self.task_row1.data_ptr(),
+                                        self.counts.data_ptr(), _lib.stream_ptr()), "ent2rel_plan")
+        self.pos = torch.empty(n, dtype=torch.int64, device=dev)
+        _lib.check(lib.spk_ent2rel_positions(self.keys.data_ptr(), self.vals.data_ptr(), n, self.n_rel,
+                                             self.segptr.data_ptr(), self.rel2group.data_ptr(),
+                                             self.group_tile0.data_ptr(), self.pos.data_ptr(), _lib.stream_ptr()),
+                   "ent2rel_positions")
+
+
+class PaddedRowsFn(torch.autograd.Function):
+    """X[p] = table[ids[j]] at the padded row p = pos[j] of every row j (ids None: table[j]); pad rows are zero.
+    Backward: the real rows' gradients back in input order, summed per table row by sorted segments (deterministic)."""
 
     @staticmethod
-    def forward(ctx, Xs, W, rel_sorted_ids, offsets):
-        Xs = SF.tc_friendly(Xs.contiguous())
-        d_out = W.shape[2]
-        Y = torch.empty(Xs.shape[0], (d_out + 3) // 4 * 4, dtype=torch.float32, device=Xs.device)[:, :d_out]
-        for r, lo, hi in zip(rel_sorted_ids, offsets[:-1], offsets[1:]):
-            SF.gemm_nn(Xs[lo:hi], W[r], out=Y[lo:hi])
-        ctx.save_for_backward(Xs, W)
-        ctx.seg = (rel_sorted_ids, offsets)
-        return Y
+    def forward(ctx, table, lay, ids):
+        t = table.detach()
+        t = t if t.stride(1) == 1 else t.contiguous()
+        width = t.shape[1]
+        out = torch.empty(lay.max_rows, _ld4(width), dtype=torch.float32, device=t.device)[:, :width]
+        _lib.check(_lib.load().spk_ent2rel_gather(_lib.ptr(t), t.stride(0), t.shape[0], _lib.ptr(ids), lay.vals.data_ptr(),
+                                                  lay.segptr.data_ptr(), lay.group_rel.data_ptr(),
+                                                  lay.group_tile0.data_ptr(), lay.tile_group.data_ptr(),
+                                                  lay.counts.data_ptr(), width, lay.max_rows, out.data_ptr(),
+                                                  out.stride(0), lay.err.data_ptr(), _lib.stream_ptr()), "ent2rel_gather")
+        ctx.lay, ctx.ids, ctx.n_table = lay, ids, t.shape[0]
+        return out
 
     @staticmethod
     def backward(ctx, g):
-        Xs, W = ctx.saved_tensors
-        rel_ids, offsets = ctx.seg
-        g = SF.tc_friendly(g.contiguous())
-        dX = None
+        lay, ids = ctx.lay, ctx.ids
+        g = g if g.stride(1) == 1 else g.contiguous()
+        rows = _gather_concat([(g, lay.pos, 1)], lay.n_rows, g.shape[1])
+        if ids is None:
+            return rows, None, None
+        edge = torch.stack((ids, ids), dim=0)
+        return SpecialSpmmFunctionFinal.apply(edge, rows, ctx.n_table, ids.numel(), g.shape[1]), None, None
+
+
+class GroupedProjectFn(torch.autograd.Function):
+    """Y = tanh(X_g . W[r_g]) for every group g of a RelationLayout (X padded, pad rows zero -> Y pad rows zero):
+    one grouped tcgen05 GEMM with the tanh epilogue. Backward: dZ = dY (1 - Y^2); dX_g = dZ_g . W[r_g]^T (the same
+    grouped GEMM reading W untransposed); dW[r] = X_g^T dZ_g as (relation, row chunk) tasks added in task order, exact
+    zeros for relations without rows. No host synchronisation and no per-relation launches."""
+
+    @staticmethod
+    def forward(ctx, X, W, lay):
+        lib = _lib.load()
+        w = W.detach()
+        w = w if w.is_contiguous() else w.contiguous()
+        n_rel, k, n = w.shape
+        assert X.shape == (lay.max_rows, k) and X.stride(1) == 1 and n_rel == lay.n_rel
+        Y = torch.empty(lay.max_rows, _ld4(n), dtype=torch.float32, device=X.device)[:, :n]
+        ws = torch.empty(lib.spk_gemm_nn_tc_grouped_workspace_floats(lay.max_groups, n, k), dtype=torch.float32,
+                         device=X.device)
+        _lib.check(lib.spk_gemm_nn_tc_grouped(_lib.ptr(X), X.stride(0), lay.max_rows, _lib.ptr(w), k * n, 1, n, n, k,
+                                              lay.group_rel.data_ptr(), lay.counts.data_ptr(), lay.max_groups,
+                                              lay.tile_group.data_ptr(), Y.data_ptr(), Y.stride(0), 2, ws.data_ptr(),
+                                              _lib.stream_ptr()), "gemm_nn_tc_grouped")
+        ctx.save_for_backward(X, w, Y)
+        ctx.lay = lay
+        return Y
+
+    @staticmethod
+    def backward(ctx, dY):
+        lib = _lib.load()
+        X, w, Y = ctx.saved_tensors
+        lay = ctx.lay
+        n_rel, k, n = w.shape
+        dev = X.device
+        dY = dY if dY.stride(1) == 1 else dY.contiguous()
+        dZ = torch.empty(lay.max_rows, _ld4(n), dtype=torch.float32, device=dev)[:, :n]
+        _lib.check(lib.spk_tanh_bwd(Y.data_ptr(), Y.stride(0), dY.data_ptr(), dY.stride(0), lay.max_rows, n,
+                                    dZ.data_ptr(), dZ.stride(0), _lib.stream_ptr()), "tanh_bwd")
+        dX = dW = None
         if ctx.needs_input_grad[0]:
-            dX = torch.empty(Xs.shape[0], (Xs.shape[1] + 3) // 4 * 4, dtype=torch.float32, device=Xs.device)[:, :Xs.shape[1]]
-        dW = torch.zeros_like(W) if ctx.needs_input_grad[1] else None
-        for r, lo, hi in zip(rel_ids, offsets[:-1], offsets[1:]):
-            if dX is not None:
-                SF.gemm_nn(g[lo:hi], W[r].t().contiguous(), out=dX[lo:hi])
-            if dW is not None:
-                SF.gemm_tn(Xs[lo:hi], g[lo:hi], out=dW[r])
-        return dX, dW, None, None
+            dX = torch.empty(lay.max_rows, _ld4(k), dtype=torch.float32, device=dev)[:, :k]
+            ws = torch.empty(lib.spk_gemm_nn_tc_grouped_workspace_floats(lay.max_groups, k, n), dtype=torch.float32,
+                             device=dev)
+            _lib.check(lib.spk_gemm_nn_tc_grouped(dZ.data_ptr(), dZ.stride(0), lay.max_rows, w.data_ptr(), k * n, n, 1, k,
+                                                  n, lay.group_rel.data_ptr(), lay.counts.data_ptr(), lay.max_groups,
+                                                  lay.tile_group.data_ptr(), dX.data_ptr(), dX.stride(0), 0,
+                                                  ws.data_ptr(), _lib.stream_ptr()), "gemm_nn_tc_grouped")
+        if ctx.needs_input_grad[1]:
+            dW = torch.empty(n_rel, k, n, dtype=torch.float32, device=dev)
+            ws = torch.empty(max(1, lib.spk_gemm_tn_tc_grouped_workspace_floats(lay.max_tasks, k, n)),
+                             dtype=torch.float32, device=dev)
+            _lib.check(lib.spk_gemm_tn_tc_grouped(X.data_ptr(), X.stride(0), dZ.data_ptr(), dZ.stride(0), lay.max_rows,
+                                                  k, n, lay.task_row0.data_ptr(), lay.task_row1.data_ptr(),
+                                                  lay.counts.data_ptr(), lay.max_tasks, lay.rel2group.data_ptr(),
+                                                  lay.task_ptr.data_ptr(), n_rel, dW.data_ptr(), ws.data_ptr(),
+                                                  _lib.stream_ptr()), "gemm_tn_tc_grouped")
+        return dX, dW, None
 
 
 def ent2rel_project(rows, w_ent2rel, rel_ids):
-    """tanh(rows[b] . W_ent2rel[rel_ids[b]]) (GAT_sep_space/models.py:316-320): triples are grouped by relation (stable
-    sort of the ids), each group is one tensor-core GEMM against its relation's matrix, results return to input order."""
-    rel_ids = rel_ids.to(rows.device)
-    order = torch.sort(rel_ids, stable=True).indices
-    counts = torch.bincount(rel_ids, minlength=w_ent2rel.shape[0]).tolist()
-    present = [r for r, c in enumerate(counts) if c]
-    offsets = [0]
-    for r in present:
-        offsets.append(offsets[-1] + counts[r])
-    xs = GatherRowsFn.apply(rows, order)
-    ys = TanhFn.apply(_GroupedMatMulFn.apply(xs, w_ent2rel, present, offsets))
-    inv = torch.empty_like(order)
-    inv[order] = torch.arange(order.numel(), device=order.device)
-    return GatherRowsFn.apply(ys, inv)
+    """tanh(rows[b] . W_ent2rel[rel_ids[b]]) (GAT_sep_space/models.py:316-320): rows grouped by relation on the device
+    (RelationLayout), one grouped tensor-core GEMM for all relations, results back in input order."""
+    rel_ids = rel_ids.to(device=rows.device, dtype=torch.int64).contiguous()
+    n = rel_ids.numel()
+    if n == 0:
+        return rows.new_empty(0, w_ent2rel.shape[2])
+    lay = RelationLayout(rel_ids, n, 1, 1, w_ent2rel.shape[0])
+    y = GroupedProjectFn.apply(PaddedRowsFn.apply(rows, lay, None), w_ent2rel, lay)
+    out = GatherRowsFn.apply(y, lay.pos)
+    if int(lay.err.item()):
+        raise IndexError("relation id out of range for W_ent2rel")
+    return out
 
 
 class ConvKB(nn.Module):

@@ -104,6 +104,8 @@ struct TcParams {
     int raw_hi;                                 // the MMA reads the raw fp32 tile as "hi" (kind::tf32 ignores the low 13 mantissa bits)
     int cs;                                     // cluster size (1 or 2): the CTAs of a cluster work on consecutive M tiles of the
                                                 // same N tile in lock-step and share every weight tile by TMA multicast
+    const int* tile_group;                      // grouped kernel only: group of every 128-row M tile; the weight rows of group g
+    const int* n_mtiles;                        // start at row g * N of the stacked B_hi / B_lo; *n_mtiles = M tiles to run
 };
 
 // ELU(x) = x (x > 0) else expm1(x); same evaluation as the edge kernels (degree-5 polynomial near 0)
@@ -118,6 +120,9 @@ __device__ __forceinline__ float tc_elu(float x) {
 // of tanh_fwd_kernel (spk_convkb.cu, no fast-math), so act = 2 gives the same bits as the product followed by spk_tanh_fwd.
 __device__ __forceinline__ float tc_act(float x, int act) { return act == 2 ? tanhf(x) : tc_elu(x); }
 
+// GROUPED: C_g = A_g . B_g for row groups padded to whole M tiles (spk_ent2rel_*): the tile count and each tile's group are
+// read from the device, so the launch needs no host-side knowledge of the grouping (cs == 1 only)
+template <bool GROUPED>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmBhi,
                   const __grid_constant__ CUtensorMap tmBlo, const __grid_constant__ CUtensorMap tmC, const TcParams p) {
@@ -148,7 +153,7 @@ gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     const int cs = p.cs;
     const uint32_t crank = cs > 1 ? cluster_ctarank() : 0u;
     const uint16_t cmask = (uint16_t)((1u << cs) - 1u);
-    const long total = ((m_tiles + cs - 1) / cs) * p.n_tiles_n;
+    const long total = GROUPED ? (long)*p.n_mtiles * p.n_tiles_n : ((m_tiles + cs - 1) / cs) * p.n_tiles_n;
     const long first = blockIdx.x / cs, stride = gridDim.x / cs;
     const uint32_t b_slice = b_tile / (uint32_t)cs;               // bytes of this CTA's share of a weight tile
     const int b_rows = p.BN / cs;
@@ -175,7 +180,8 @@ gemm_nn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         if (lane == 0) {                                           // ---- TMA producer
             uint32_t it = 0;
             for (long tile = first; tile < total; tile += stride) {
-                const int m0 = (int)((tile / p.n_tiles_n) * cs + crank) * TC_BM, n0 = (int)(tile % p.n_tiles_n) * p.BN;
+                const int m0 = (int)((tile / p.n_tiles_n) * cs + crank) * TC_BM;
+                const int n0 = (int)(tile % p.n_tiles_n) * p.BN + (GROUPED ? p.tile_group[tile / p.n_tiles_n] * p.N : 0);
                 for (int kb = 0; kb < num_kb; ++kb, ++it) {
                     const int s = it % p.stages;
                     const uint32_t ph = (it / p.stages) & 1u;
@@ -729,7 +735,7 @@ int gemm_nn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
         if (int rc = make_map(&tBh, bhi, N, K, ldt, BN / 2)) return rc;
         if (int rc = make_map(&tBl, blo, N, K, ldt, BN / 2)) return rc;
         if (int rc = make_map(&tC, C, M, N, ldc, 32)) return rc;
-        TcParams q;
+        TcParams q = {};
         q.C = C; q.ldc = ldc; q.M = M; q.N = N; q.K = K; q.BN = BN; q.n_tiles_n = n_tiles_n; q.stages = stages2;
         q.accumulate = accumulate; q.act = act; q.c_vec = c_vec; q.c_tma = 1; q.raw_hi = 1; q.cs = 2;
         static SmemLimit lim2;
@@ -765,12 +771,12 @@ int gemm_nn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
     if (c_tma) { if (int rc = make_map(&tmC, C, M, N, ldc, 32)) return rc; }
     else tmC = tmA;
 
-    TcParams p;
+    TcParams p = {};
     p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.BN = BN; p.n_tiles_n = n_tiles_n; p.stages = stages;
     p.accumulate = accumulate; p.act = act;
     p.c_vec = c_vec; p.c_tma = c_tma; p.raw_hi = tc_raw_hi(); p.cs = cs;
     static SmemLimit lim;
-    if (lim.ensure(gemm_nn_tc_kernel, 226 * 1024) != cudaSuccess) {
+    if (lim.ensure(gemm_nn_tc_kernel<false>, 226 * 1024) != cudaSuccess) {
         set_error("gemm_tc: cannot raise dynamic shared memory limit");
         (void)cudaGetLastError();
         return 3;
@@ -789,7 +795,7 @@ int gemm_nn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
         static int clusters[64] = {};
         int nc = (dev >= 0 && dev < 64) ? clusters[dev] : 0;
         if (nc == 0) {
-            if (cudaOccupancyMaxActiveClusters(&nc, gemm_nn_tc_kernel, &cfg) != cudaSuccess || nc < 1) { (void)cudaGetLastError(); nc = sms / cs / 2; }
+            if (cudaOccupancyMaxActiveClusters(&nc, gemm_nn_tc_kernel<false>, &cfg) != cudaSuccess || nc < 1) { (void)cudaGetLastError(); nc = sms / cs / 2; }
             if (dev >= 0 && dev < 64) clusters[dev] = nc;
         }
         resident = (long)nc * cs;
@@ -798,7 +804,7 @@ int gemm_nn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
     grid = grid / cs * cs;
     if (grid < (unsigned)cs) grid = (unsigned)cs;
     cfg.gridDim = dim3(grid);
-    (void)cudaLaunchKernelEx(&cfg, gemm_nn_tc_kernel, tmA, tmBhi, tmBlo, tmC, p);
+    (void)cudaLaunchKernelEx(&cfg, gemm_nn_tc_kernel<false>, tmA, tmBhi, tmBlo, tmC, p);
     return check_launch("gemm_nn_tc");
 }
 
@@ -830,6 +836,9 @@ __device__ __forceinline__ uint64_t make_mnmajor_sw128_desc(uint32_t saddr) {
 struct TnParams {
     float* part; long M; int Ka; int Nb; int BN; int n_tiles_n; int n_tiles_k; int splits; long m_per_split; int stages;
     int raw_hi;
+    const int* task_row0;                       // grouped kernel only: split z covers rows [task_row0[z], task_row1[z]) and
+    const int* task_row1;                       // runs when z < *n_tasks
+    const int* n_tasks;
 };
 
 // Decoupled rings: the raw tiles (TMA destination; read by the MMA as the "hi" operands) live in a ring of
@@ -839,6 +848,7 @@ constexpr int TN_LO_SLOTS = 2;
 constexpr int TN_SPLIT_WARPS = 8;
 constexpr int TN_THREADS = (2 + TN_SPLIT_WARPS + 4) * 32;      // TMA, MMA, splitters, epilogue
 
+template <bool GROUPED>
 __global__ void __launch_bounds__(TN_THREADS, 1)
 gemm_tn_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmG, const TnParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -861,9 +871,10 @@ gemm_tn_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant
 
     const int tile = blockIdx.x % (p.n_tiles_k * p.n_tiles_n);
     const int split = blockIdx.x / (p.n_tiles_k * p.n_tiles_n);
+    if (GROUPED && split >= *p.n_tasks) return;                    // (the grid is sized for the largest task count)
     const int ka0 = (tile / p.n_tiles_n) * 128, nb0 = (tile % p.n_tiles_n) * p.BN;
-    const long mbeg = (long)split * p.m_per_split;
-    long mend = mbeg + p.m_per_split;
+    const long mbeg = GROUPED ? (long)p.task_row0[split] : (long)split * p.m_per_split;
+    long mend = GROUPED ? (long)p.task_row1[split] : mbeg + p.m_per_split;
     if (mend > p.M) mend = p.M;
     const int num_kb = mend > mbeg ? (int)((mend - mbeg + TN_BKM - 1) / TN_BKM) : 0;
 
@@ -1047,21 +1058,146 @@ int gemm_tn_tc(const float* A, long lda, const float* B, long ldb, float* C, lon
     CUtensorMap tmX, tmG;
     if (int rc = make_map_tn(&tmX, A, M, Ka, lda)) return rc;
     if (int rc = make_map_tn(&tmG, B, M, Nb, ldb)) return rc;
-    TnParams p;
+    TnParams p = {};
     p.part = workspace; p.M = M; p.Ka = Ka; p.Nb = Nb; p.BN = pl.BN; p.n_tiles_n = pl.n_tiles_n; p.n_tiles_k = pl.n_tiles_k;
     p.splits = pl.splits; p.m_per_split = pl.m_per_split; p.stages = pl.stages; p.raw_hi = tc_raw_hi();
     static SmemLimit lim;
-    if (lim.ensure(gemm_tn_tc_kernel, 226 * 1024) != cudaSuccess) {
+    if (lim.ensure(gemm_tn_tc_kernel<false>, 226 * 1024) != cudaSuccess) {
         set_error("gemm_tn_tc: cannot raise dynamic shared memory limit");
         (void)cudaGetLastError();
         return 3;
     }
     const unsigned grid = (unsigned)(pl.n_tiles_k * pl.n_tiles_n * pl.splits);
-    gemm_tn_tc_kernel<<<grid, TN_THREADS, pl.smem, s>>>(tmX, tmG, p);
+    gemm_tn_tc_kernel<false><<<grid, TN_THREADS, pl.smem, s>>>(tmX, tmG, p);
     if (int rc = check_launch("gemm_tn_tc")) return rc;
     const long elems = (long)Ka * Nb;
     tn_reduce_tc_kernel<<<(unsigned)((elems + 255) / 256), 256, 0, s>>>(workspace, pl.splits, elems, Nb, C, ldc, accumulate);
     return check_launch("tn_reduce_tc");
+}
+
+// ------------------------------------------------------------------------------------------------
+// Grouped products for the relation-space projection of the GAT_sep_space variant (spk_ent2rel_*):
+// rows grouped by relation, every group padded with zero rows to whole 128-row M tiles, group g
+// multiplying by its own weight W[group_rel[g]]. Group count, tile table and task table live on the
+// device; the host sizes grids and buffers for the worst case and never reads them back.
+// ------------------------------------------------------------------------------------------------
+namespace {
+
+// Bt_hi / Bt_lo of every present group, stacked: row g * N + n, column k < ldt holds split(W[r][k-th element of the
+// n-th output column]) = W[r * rstride + n * sn + k * sk] (zero for k >= K). sn = 1, sk = N reads W[r] as B [K, N]
+// (transposed into K-major); sn = ldw, sk = 1 reads it as B^T, i.e. multiplies by W[r]^T (no transpose).
+__global__ void tc_prepare_b_grouped_kernel(const float* __restrict__ W, long rstride, long sn, long sk, int K, int N,
+                                            const int* __restrict__ group_rel, const int* __restrict__ n_groups,
+                                            float* __restrict__ hi, float* __restrict__ lo, int ldt) {
+    const long per = (long)N * ldt;
+    const long total = (long)*n_groups * per;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+        const long g = i / per, rem = i % per;
+        const int n = (int)(rem / ldt), k = (int)(rem % ldt);
+        const float x = k < K ? W[(long)group_rel[g] * rstride + n * sn + k * sk] : 0.f;
+        const float h = __uint_as_float(__float_as_uint(x) & 0xffffe000u);
+        hi[i] = h;
+        lo[i] = x - h;
+    }
+}
+
+// dW[r] = sum of the partials of group rel2group[r]'s tasks, in task order (zeros for a relation without rows)
+__global__ void tn_reduce_grouped_kernel(const float* __restrict__ part, const int* __restrict__ rel2group,
+                                         const int* __restrict__ task_ptr, long elems, int n_rel, float* __restrict__ C) {
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= elems * n_rel) return;
+    const int r = (int)(i / elems);
+    const long idx = i % elems;
+    const int g = rel2group[r];
+    float s = 0.f;
+    if (g >= 0)
+        for (int z = task_ptr[g]; z < task_ptr[g + 1]; ++z) s += part[(long)z * elems + idx];
+    C[i] = s;
+}
+
+}  // namespace
+
+int gemm_nn_tc_grouped(const float* A, long lda, long max_rows, const float* W, long rstride, long sn, long sk,
+                       int N, int K, const int* group_rel, const int* n_groups, int max_groups, const int* tile_group,
+                       const int* n_mtiles, float* C, long ldc, int act, float* workspace, cudaStream_t s) {
+    const int ldt = gemm_tc_ldt(K);
+    float* bhi = workspace;
+    float* blo = workspace + (long)max_groups * N * ldt;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long nb = (long)max_groups * N * ldt;
+    long pblocks = (nb + 255) / 256;
+    if (pblocks > 8L * sms) pblocks = 8L * sms;
+    tc_prepare_b_grouped_kernel<<<(unsigned)(pblocks > 0 ? pblocks : 1), 256, 0, s>>>(W, rstride, sn, sk, K, N, group_rel,
+                                                                                     n_groups, bhi, blo, ldt);
+    if (int rc = check_launch("tc_prepare_b_grouped")) return rc;
+
+    // tile shape, epilogue and pipeline depth exactly as gemm_nn_tc, so a group's rows come out as that kernel gives them
+    const int n_tiles_n = (N + 255) / 256;
+    const int bn_round = n_tiles_n > 1 ? 32 : 16;
+    int BN = ((N + n_tiles_n - 1) / n_tiles_n + bn_round - 1) / bn_round * bn_round;
+    if (BN < 16) BN = 16;
+    const int stage_bytes = 2 * TC_A_TILE + 2 * BN * 128;
+    const int c_vec = (ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(C) & 15) == 0);
+    const int c_tma = c_vec && (N % 4 == 0);
+    const int staging = c_tma ? 4 * 8192 : 0;
+    int stages = (225 * 1024 - 1024 - staging) / stage_bytes;
+    if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
+    if (stages < 1) { set_error("gemm_tc_grouped: tile does not fit shared memory"); return 3; }
+    const int smem = stages * stage_bytes + staging + 1024;
+
+    CUtensorMap tmA, tmBhi, tmBlo, tmC;
+    if (int rc = make_map(&tmA, A, max_rows, K, lda, TC_BM)) return rc;
+    if (int rc = make_map(&tmBhi, bhi, (long)max_groups * N, K, ldt, BN)) return rc;
+    if (int rc = make_map(&tmBlo, blo, (long)max_groups * N, K, ldt, BN)) return rc;
+    if (c_tma) { if (int rc = make_map(&tmC, C, max_rows, N, ldc, 32)) return rc; }
+    else tmC = tmA;
+
+    TcParams p = {};
+    p.C = C; p.ldc = ldc; p.M = max_rows; p.N = N; p.K = K; p.BN = BN; p.n_tiles_n = n_tiles_n; p.stages = stages;
+    p.accumulate = 0; p.act = act; p.c_vec = c_vec; p.c_tma = c_tma; p.raw_hi = tc_raw_hi(); p.cs = 1;
+    p.tile_group = tile_group; p.n_mtiles = n_mtiles;
+    static SmemLimit lim;
+    if (lim.ensure(gemm_nn_tc_kernel<true>, 226 * 1024) != cudaSuccess) {
+        set_error("gemm_tc_grouped: cannot raise dynamic shared memory limit");
+        (void)cudaGetLastError();
+        return 3;
+    }
+    const long max_tiles = (max_rows + TC_BM - 1) / TC_BM * n_tiles_n;
+    const unsigned grid = (unsigned)(max_tiles < sms ? (max_tiles > 0 ? max_tiles : 1) : sms);
+    gemm_nn_tc_kernel<true><<<grid, TC_THREADS, smem, s>>>(tmA, tmBhi, tmBlo, tmC, p);
+    return check_launch("gemm_nn_tc_grouped");
+}
+
+long gemm_tn_tc_grouped_workspace_floats(int max_tasks, int Ka, int Nb) { return (long)max_tasks * Ka * Nb; }
+
+int gemm_tn_tc_grouped(const float* A, long lda, const float* B, long ldb, long max_rows, int Ka, int Nb,
+                       const int* task_row0, const int* task_row1, const int* n_tasks, int max_tasks,
+                       const int* rel2group, const int* task_ptr, int n_rel, float* C, float* workspace, cudaStream_t s) {
+    const TnPlan pl = tn_plan(max_rows, Ka, Nb);
+    CUtensorMap tmX, tmG;
+    if (int rc = make_map_tn(&tmX, A, max_rows, Ka, lda)) return rc;
+    if (int rc = make_map_tn(&tmG, B, max_rows, Nb, ldb)) return rc;
+    TnParams p = {};
+    p.part = workspace; p.M = max_rows; p.Ka = Ka; p.Nb = Nb; p.BN = pl.BN; p.n_tiles_n = pl.n_tiles_n;
+    p.n_tiles_k = pl.n_tiles_k; p.splits = max_tasks; p.m_per_split = 0; p.stages = pl.stages; p.raw_hi = tc_raw_hi();
+    p.task_row0 = task_row0; p.task_row1 = task_row1; p.n_tasks = n_tasks;
+    static SmemLimit lim;
+    if (lim.ensure(gemm_tn_tc_kernel<true>, 226 * 1024) != cudaSuccess) {
+        set_error("gemm_tn_tc_grouped: cannot raise dynamic shared memory limit");
+        (void)cudaGetLastError();
+        return 3;
+    }
+    if (max_tasks > 0) {
+        const unsigned grid = (unsigned)(pl.n_tiles_k * pl.n_tiles_n * max_tasks);
+        gemm_tn_tc_kernel<true><<<grid, TN_THREADS, pl.smem, s>>>(tmX, tmG, p);
+        if (int rc = check_launch("gemm_tn_tc_grouped")) return rc;
+    }
+    const long elems = (long)Ka * Nb;
+    tn_reduce_grouped_kernel<<<(unsigned)((elems * n_rel + 255) / 256), 256, 0, s>>>(workspace, rel2group, task_ptr, elems,
+                                                                                     n_rel, C);
+    return check_launch("tn_reduce_grouped");
 }
 
 }  // namespace spk

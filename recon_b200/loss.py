@@ -7,6 +7,10 @@
     (default 2, main.py:68-69).
   * its backward (the gradient `SpKBGATModified`'s backward consumes) as a deterministic segmented sum over a
     radix-sorted incidence list instead of autograd's `index_put_(accumulate=True)` atomics.
+  * with `model_gat=` (the GAT_sep_space variant, GAT_sep_space/main.py:360-377) heads and tails are first projected into
+    relation space, tanh(e . W_ent2rel[r]) with each row's own relation: the 2T entity rows are gathered straight into a
+    relation-grouped, tile-padded layout, projected by one grouped tcgen05 GEMM (convkb.GroupedProjectFn), and the same
+    margin kernels run on the projected table with triples (padded head row, r, padded tail row).
   * `sgd_step(params, lr)` — `torch.optim.SGD(model.parameters(), lr).step()` (main.py:445-446, 524) in one launch.
 
 All arithmetic runs in libspkbgat (`spk_margin_loss_fwd/bwd`, `spk_triple_incidence`, `spk_sort_pairs`,
@@ -103,9 +107,30 @@ class MarginLossFn(torch.autograd.Function):
         return d_ent, d_rel, None, None, None, None
 
 
-def batch_gat_loss(gat_loss_func, train_indices, entity_embed, relation_embed, valid_invalid_ratio_gat=2):
+def _margin_loss_sep(train_indices, entity_embed, relation_embed, w_ent2rel, n_pos, margin, mean):
+    """The margin loss of GAT_sep_space/main.py:344-377: x = tanh(e_h W[r]) + rel[r] - tanh(e_t W[r]) per row."""
+    from .convkb import RelationLayout, PaddedRowsFn, GroupedProjectFn
+    if not (entity_embed.is_cuda and relation_embed.is_cuda and w_ent2rel.is_cuda):
+        raise RuntimeError("recon_b200 ops need CUDA tensors (no CPU fallback)")
+    dev = entity_embed.device
+    with torch.cuda.device(dev):
+        tri = train_indices.to(device=dev, dtype=torch.int64).contiguous()
+        t = int(tri.shape[0])
+        assert w_ent2rel.dim() == 3 and w_ent2rel.shape[1] == entity_embed.shape[1], "W_ent2rel must be [R, HD, HD']"
+        lay = RelationLayout(tri[:, 1], t, 2, 3, w_ent2rel.shape[0])     # rows: the T heads, then the T tails
+        x = PaddedRowsFn.apply(entity_embed, lay, torch.cat((tri[:, 0], tri[:, 2])))
+        y = GroupedProjectFn.apply(x, w_ent2rel, lay)
+        syn = torch.stack((lay.pos[:t], tri[:, 1], lay.pos[t:]), dim=1)
+        loss, err = MarginLossFn.apply(y, relation_embed, syn, n_pos, margin, mean)
+        return loss, err | lay.err
+
+
+def batch_gat_loss(gat_loss_func, train_indices, entity_embed, relation_embed, valid_invalid_ratio_gat=2, *,
+                   model_gat=None):
     """Drop-in for GAT/main.py:344-376. `gat_loss_func` is the reference's `nn.MarginRankingLoss(margin=...)`
-    (only its `margin` and `reduction` are read); `train_indices` int64 [T,3], positives first (main.py:348-349)."""
+    (only its `margin` and `reduction` are read); `train_indices` int64 [T,3], positives first (main.py:348-349).
+    `model_gat`: any object with `.W_ent2rel` [R, HD, HD] selects the GAT_sep_space loss (main.py:360-377), whose
+    gradient also reaches W_ent2rel (exact zeros for relations without rows)."""
     ratio = int(valid_invalid_ratio_gat)
     t = int(train_indices.shape[0])
     len_pos_triples = int(t / (ratio * 2 + 1))                                    # main.py:345-346
@@ -116,8 +141,12 @@ def batch_gat_loss(gat_loss_func, train_indices, entity_embed, relation_embed, v
     reduction = getattr(gat_loss_func, "reduction", "mean")
     if reduction not in ("mean", "sum"):
         raise NotImplementedError("batch_gat_loss: reduction must be 'mean' (the reference's) or 'sum'")
-    loss, err = MarginLossFn.apply(entity_embed, relation_embed, train_indices, len_pos_triples, margin,
-                                   reduction == "mean")
+    if model_gat is not None:
+        loss, err = _margin_loss_sep(train_indices, entity_embed, relation_embed, model_gat.W_ent2rel, len_pos_triples,
+                                     margin, reduction == "mean")
+    else:
+        loss, err = MarginLossFn.apply(entity_embed, relation_embed, train_indices, len_pos_triples, margin,
+                                       reduction == "mean")
     if int(err.item()) != 0:                                                      # the reference's gathers (main.py:353-355)
         raise IndexError("train_indices out of range for the entity / relation embedding tables")
     assert not bool(torch.isnan(loss).any()), "batch_gat_loss: NaN loss"          # main.py:374 (the reference syncs here too)
