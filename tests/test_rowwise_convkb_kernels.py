@@ -23,10 +23,11 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from helpers import B200_SMS, gemm_nn_branch
+
 U = 2.0 ** -24                    # fp32 unit roundoff
 EPS = 1e-12                       # F.normalize's eps (models.py:160-161, 175-179)
 RK_REG = 16                       # spk_convkb.cu: rank_scores keeps a row in RK_REG 32-float register chunks
-B200_SMS = 148                    # SM count the GEMM's pair / cluster thresholds are computed from on a B200
 LRELU_SLOPE = 0.01                # convkb.LRELU_SLOPE, nn.LeakyReLU()'s default
 SENTINEL = -1234.5                # fills every padding column and every row past n; no kernel here writes it
 
@@ -48,24 +49,6 @@ def spmm_branch(width):
 def rank_scores_rc(d):
     """spk_convkb.cu launch_rank_scores: a pair row lives in RK_REG register chunks of 32 floats; wider rows are code 2."""
     return 0 if d <= 32 * RK_REG else 2
-
-
-def gemm_nn_branch(m, n, lda, ldc, accumulate, act, path, sms=B200_SMS):
-    """(kernel, epilogue) of functional.gemm_nn(act=act) for a 16-byte aligned A / C allocation: the SIMT GEMM followed by
-    spk_elu_inplace, or spk_gemm_tc.cu gemm_nn_tc (TMA-store epilogue when c_vec && !(act && accumulate), else the
-    per-thread-row epilogue, float4 when C allows it), its pair-CTA kernel (SPK_TC_PAIR=1) or 2-CTA clusters
-    (SPK_TC_CLUSTER=2), both only once there are 2 x sms tiles of 128 rows. TMA stores only whole rows of 16-byte
-    units, so N % 4 != 0 takes the per-thread-row epilogue. BN is always a multiple of 16 and the raw tile is the hi
-    operand by default, so the pair kernel's other conditions always hold."""
-    if path == "simt" or n > 512 or lda % 4:
-        return "simt", "elu_inplace"
-    c_vec = ldc % 4 == 0
-    c_tma = c_vec and n % 4 == 0 and not (act and accumulate)
-    tiles = (m + 127) // 128 * ((n + 255) // 256)
-    if path == "tc-pair" and c_tma and tiles >= 2 * sms:
-        return "pair", "tma"
-    cluster = path == "tc-cluster" and not accumulate and tiles >= 2 * sms
-    return "cluster" if cluster else "tc", "tma" if c_tma else "row-vec4" if c_vec else "row-scalar"
 
 
 ROWNORM_WIDTHS = [1, 2, 7, 50, 63, 64, 66, 200, 255, 256, 258, 400, 512]
